@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N --steps K --warmup W]                 our engine (1 process per GPU)
   python bench.py --impl reference [...]                          grab master (PCRE2-JIT shim) on the host cores
+  python bench.py [...] --dump-outputs DIR                        also writes the records of the last timed step as .npy
 
 One JSON line on stdout (rank 0).  The headline (`value`, `roofline`, `e2e`, `cpu_baseline`) is BASELINE.json configs[1]:
 a literal (-S semantics) over a synthetic corpus of 1 MiB files, 64 GiB per GPU, device resident, all offsets (-O -l).
@@ -37,6 +38,7 @@ PATTERN = "foobardoesexist"      # literal; planted once per 64 files (= per 64 
 NEEDLE_EVERY = 64
 SEED = 2
 FILE_LEN = 1 << 20
+DUMP_BYTES = 60 * MiB  # what --dump-outputs writes at most (64 MB with the .npy headers)
 REF_BIN = os.path.join(ROOT, "oracle", "_ref", "grab_ref")
 ENGINE_LABEL = "grab master + PCRE2 10.42 JIT via oracle/shim (NOT hyperscan: no -H source or library available)"
 
@@ -181,6 +183,24 @@ class records_by_file:
 
     def __len__(self):
         return len(self.fid)
+
+
+def dump_records(r, out_dir, prefix, max_bytes):
+    """The records a caller of the scan receives, one float64 array per field (exact: offsets and ids stay below 2**53),
+    so that two builds can be compared field for field.  Above `max_bytes` a fixed-seed sample of the records is written,
+    with the sampled row numbers as `sample_rows`."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    fields = ("file_id", "start", "match_len")
+    rows = None
+    if len(r) * 8 * len(fields) > max_bytes:
+        keep = max_bytes // (8 * (len(fields) + 1))
+        rows = np.sort(np.random.default_rng(0).choice(len(r), size=keep, replace=False))
+        r = r[rows]
+        np.save(os.path.join(out_dir, prefix + "sample_rows.npy"), rows.astype(np.float64))
+    for f in fields:
+        np.save(os.path.join(out_dir, prefix + f + ".npy"), r[f].astype(np.float64))
+    log("bench: wrote %d%s records to %s" % (len(r), "" if rows is None else " sampled", out_dir))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -394,7 +414,11 @@ def main():
     ap.add_argument("--config-steps", type=int, default=5, help="timed steps of each entry of `configs`")
     ap.add_argument("--only", default="", help="comma list of config indices to run in `configs` (default: all)")
     ap.add_argument("--quick", action="store_true", help="skip the cpu baselines and the e2e legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the records of the headline's last timed step to DIR/<field>.npy "
+                    "(float64; a seeded sample of the records above %d MiB in all)" % (DUMP_BYTES // MiB))
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -429,8 +453,9 @@ def main():
     scale = min(1.0, a.corpus_gib / 64.0)
     buf_bytes = int(64 * GiB * scale)
     if buf_bytes > free_b - 12 * GiB:
-        buf_bytes = max(GiB, free_b - 12 * GiB)
-        scale = buf_bytes / (64.0 * GiB)
+        # the corpus is never shrunk to fit: the arguments alone fix the workload, so that runs stay comparable
+        sys.exit("bench: a %.1f GiB corpus and 12 GiB of working memory do not fit in the %.1f GiB free on GPU %d: "
+                 "pass a smaller --corpus-gib" % (buf_bytes / GiB, free_b / GiB, local_rank))
     dptr = ctx.device_alloc(buf_bytes)
     peaks = {}
     try:
@@ -533,6 +558,8 @@ def main():
     # the oracle on >= 64 regenerated files ----
     import corpus
     r = r.copy()
+    if a.dump_outputs:
+        dump_records(r, a.dump_outputs, "" if world == 1 else "rank%d_" % rank, DUMP_BYTES // world)
     ids = np.arange(first_id, first_id + n_files)
     planted = ids[ids % NEEDLE_EVERY == NEEDLE_EVERY // 2]
     want = {int(f): corpus.needle_offset(SEED, int(f), FILE_LEN, len(PATTERN)) for f in planted}

@@ -9,12 +9,16 @@ pin for both the oracle port (oracle/grab_oracle.c) and the CUDA engine.  Run fr
     make -C oracle ref && python tests/golden/make_golden.py [--big]
 
 --big also regenerates big.json (Appendix B.2 / B.3: 40 MiB and 256 MiB inputs; ~1 min).
+ref_stdout.json.gz and host_ref.json hold the reference's output on the inputs that tests/test_oracle_vs_ref.py and
+tests/test_hostcheck.py generate (seeded): those tests compare with these recordings instead of running the reference.
 """
 import base64
 import ctypes
+import gzip
 import hashlib
 import json
 import os
+import pathlib
 import random
 import subprocess
 import sys
@@ -22,6 +26,7 @@ import tempfile
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
+sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 import corpus  # noqa: E402
 
@@ -319,6 +324,61 @@ def gen_big():
     return out
 
 
+# --------------------------------------------------------------------------------------------
+# 5. the reference's output on the seeded inputs of test_oracle_vs_ref.py and test_hostcheck.py
+# --------------------------------------------------------------------------------------------
+def gen_ref_stdout():
+    """Runs each test of test_oracle_vs_ref.py once with its lookup of the recording replaced by a run of the reference,
+    so the recording holds exactly the (pattern, flags, input) triples the tests ask for."""
+    import test_oracle_vs_ref as T
+    rows = {}
+
+    def run(pattern, data, flags=("-O", "-l")):
+        k = (pattern, tuple(flags), T.input_key(data))
+        with tempfile.NamedTemporaryFile() as f:
+            f.write(data)
+            f.flush()
+            try:
+                p = subprocess.run([REF] + list(flags) + [pattern, f.name], stdout=subprocess.PIPE, stderr=subprocess.PIPE,
+                                   timeout=T.REF_TIMEOUT_S)
+            except subprocess.TimeoutExpired:
+                rows[k] = None
+                raise
+        assert p.returncode == 0, p.stderr
+        rows[k] = T.digest(p.stdout)
+        return rows[k]
+
+    T.ref_stdout = run
+    for name in ("test_random_patterns_stdout_identical", "test_inline_options_ungreedy_extended_comment",
+                 "test_minlen_quirk_q1_against_reference", "test_long_lines_line_mode_against_reference"):
+        getattr(T, name)()
+    return [[pat, list(flags), key, d] for (pat, flags, key), d in sorted(rows.items(), key=lambda kv: json.dumps(kv[0]))]
+
+
+def gen_host_ref():
+    import test_hostcheck as H
+    out = {"tree": {}, "f4": {}}
+    with tempfile.TemporaryDirectory() as td:
+        H._tree(pathlib.Path(td))
+        for flags in H.TREE_FLAGS:
+            rc, so, se = run_ref(flags + ["foo|bar|baz|quux", "tree"], cwd=td)
+            assert rc == 0, se
+            out["tree"][" ".join(flags)] = H.sorted_lines_digest(so)
+    with tempfile.TemporaryDirectory() as td:
+        fn = os.path.join(td, "big.bin")
+        H._f4_file(fn)
+        for flags in H.F4_FLAGS:
+            rc, so, se = run_ref(["-L"] * 5 + flags + ["NEEDLE", fn])
+            assert rc == 0, se
+            out["f4"][" ".join(flags)] = b64(so)
+    with tempfile.TemporaryDirectory() as td:
+        with open(os.path.join(td, "a"), "wb") as f:
+            f.write(b"xx foo yy\nzz foo\n\n")
+        rc, so, se = run_ref(["-O", "-l", "foo", "a", "nope"], cwd=td)
+        out["good_then_missing"] = {"rc": rc, "stdout": b64(so), "stderr": b64(se)}
+    return out
+
+
 def main():
     if not os.path.exists(REF):
         sys.exit("build the reference first: make -C oracle ref")
@@ -326,6 +386,12 @@ def main():
         json.dump(gen_small(), f, indent=0)
     with open(os.path.join(HERE, "minlen.json"), "w") as f:
         json.dump(gen_minlen(), f, indent=0)
+    rows = gen_ref_stdout()
+    with open(os.path.join(HERE, "ref_stdout.json.gz"), "wb") as f:
+        f.write(gzip.compress(json.dumps(rows, indent=0).encode(), 9, mtime=0))
+    host = gen_host_ref()
+    with open(os.path.join(HERE, "host_ref.json"), "w") as f:
+        json.dump(host, f, indent=1)
     if "--big" in sys.argv:
         with open(os.path.join(HERE, "big.json"), "w") as f:
             json.dump(gen_big(), f, indent=0)

@@ -66,3 +66,26 @@ def test_mismatch_on_one_rank_is_seen_by_all():
 def test_failure_on_one_rank_drops_the_number_without_hanging():
     assert _run("raise") == {0: None, 1: None}
     assert _run("setup_failed") == {0: None, 1: None}
+
+
+def test_dump_records_exact_and_bounded(tmp_path):
+    """--dump-outputs: every field as exact float64; above the byte budget a fixed-seed sample of rows, the same one on
+    every run, within the budget."""
+    sys.path.insert(0, ROOT)
+    import bench
+    from grab_b200 import MATCH_DTYPE
+    r = np.zeros(1000, dtype=MATCH_DTYPE)
+    r["start"] = np.arange(1000, dtype=np.uint64) * np.uint64(1 << 40) + np.uint64(7)
+    r["file_id"] = np.arange(1000) * 3
+    r["match_len"] = 15
+    bench.dump_records(r, str(tmp_path / "all"), "", 1 << 20)
+    for f in ("start", "file_id", "match_len"):
+        got = np.load(tmp_path / "all" / (f + ".npy"))
+        assert got.dtype == np.float64 and np.array_equal(got.astype(np.uint64), r[f])
+    assert not (tmp_path / "all" / "sample_rows.npy").exists()
+    for d in ("s1", "s2"):
+        bench.dump_records(r, str(tmp_path / d), "", 3200)
+    rows = np.load(tmp_path / "s1" / "sample_rows.npy")
+    assert len(rows) == 100 and np.array_equal(rows, np.load(tmp_path / "s2" / "sample_rows.npy"))
+    assert np.array_equal(np.load(tmp_path / "s1" / "start.npy").astype(np.uint64), r["start"][rows.astype(np.int64)])
+    assert sum(os.path.getsize(tmp_path / "s1" / f) - 128 for f in os.listdir(tmp_path / "s1")) <= 3200

@@ -1,10 +1,13 @@
 """Host side of the product on a box WITHOUT a GPU: grab_b200/host (FileGrep mirror, batching, scan lanes, output
 sequencer, command line) linked against a test double of the engine ABI (tests/hostcheck/gscan_double.c, which
 answers gscan_scan_batch() with the CPU oracle).  Expected bytes are the ones recorded from the unmodified
-reference binary (tests/golden/kat.json) or produced by it / by the oracle's FileGrep::find restatement here.
+reference binary (tests/golden/kat.json, tests/golden/host_ref.json) or produced by the oracle's FileGrep::find
+restatement here.
 
 The double is test infrastructure: grab_b200/bin/grab-b200 links libgscan.so and fails loudly without a GPU."""
 import base64
+import functools
+import hashlib
 import json
 import os
 import subprocess
@@ -19,7 +22,6 @@ ROOT = os.path.dirname(HERE)
 KAT = json.load(open(os.path.join(HERE, "golden", "kat.json")))
 BUILD = os.path.join(HERE, "_build")
 BIN = os.path.join(BUILD, "grab-hostcheck")
-REF = os.path.join(ROOT, "oracle", "_ref", "grab_ref")
 
 LANES = [dict(), dict(GRAB_B200_NDEV="2", GRAB_B200_LANES="2", GRAB_B200_BATCH_BYTES="1", GSCAN_DOUBLE_JITTER="1")]
 LANE_IDS = ["1lane", "2gpu_x2lanes_jitter"]
@@ -39,6 +41,12 @@ def hostcheck_binary():
     subprocess.run(["g++", "-O2", "-std=c++17", "-Wall", os.path.join(ROOT, "grab_b200", "host", "filegrep.cc"),
                     os.path.join(ROOT, "grab_b200", "host", "main.cc"), os.path.join(BUILD, "gscan_double.o"),
                     os.path.join(BUILD, "grab_oracle.o"), "-pthread", "-o", BIN], check=True)
+
+
+@functools.lru_cache(maxsize=None)
+def host_ref():
+    """The reference's output on the inputs of the tests below (written by tests/golden/make_golden.py)."""
+    return json.load(open(os.path.join(HERE, "golden", "host_ref.json")))
 
 
 def run(args, cwd=None, env=None, binary=None):
@@ -93,6 +101,11 @@ def test_host_recursive_sorted(case, lanes, tmp_path):
     assert sorted(l for l in so.split(b"\n") if l) == [base64.b64decode(l) for l in case["sorted_lines"]]
 
 
+def sorted_lines_digest(stdout):
+    """The reference's line order across files is readdir order (Q6): output is compared as a sorted multiset of lines."""
+    return hashlib.sha256(b"\n".join(sorted(stdout.split(b"\n")))).hexdigest()
+
+
 def _tree(tmp_path, n_files=300, seed=5):
     rng = np.random.default_rng(seed)
     words = [b"foo", b"bar", b"baz", b"quux", b"lorem", b"ipsum", b"dolor", b"\n", b" ", b"sit", b"\n"]
@@ -105,7 +118,10 @@ def _tree(tmp_path, n_files=300, seed=5):
     return d
 
 
-@pytest.mark.parametrize("flags", [["-r", "-O", "-l"], ["-r"], ["-r", "-O"], ["-r", "-l"], ["-r", "-s", "-O", "-l"]], ids=lambda f: "".join(f))
+TREE_FLAGS = [["-r", "-O", "-l"], ["-r"], ["-r", "-O"], ["-r", "-l"], ["-r", "-s", "-O", "-l"]]
+
+
+@pytest.mark.parametrize("flags", TREE_FLAGS, ids=lambda f: "".join(f))
 def test_host_lanes_do_not_change_stdout(flags, tmp_path):
     """Many tiny batches finishing out of order over 6 lanes on 3 'GPUs': stdout must be byte-identical to the
     single-lane run (submission order), and as a multiset of lines identical to the reference."""
@@ -118,10 +134,7 @@ def test_host_lanes_do_not_change_stdout(flags, tmp_path):
                            env=dict(GRAB_B200_NDEV="3", GRAB_B200_LANES="2", GRAB_B200_BATCH_BYTES=bb, GSCAN_DOUBLE_JITTER="1"))
         assert rc == 0, se
         assert many == one
-    if os.path.exists(REF):
-        rcr, ref, _ = run(flags + [pat, "tree"], cwd=str(tmp_path), binary=REF)
-        assert rcr == 0
-        assert sorted(one.split(b"\n")) == sorted(ref.split(b"\n"))
+    assert sorted_lines_digest(one) == host_ref()["tree"][" ".join(flags)]
 
 
 def test_host_threads_with_lanes(tmp_path):
@@ -145,16 +158,25 @@ def _big_file(path, size, needles):
     return a
 
 
-@pytest.mark.parametrize("flags", [["-O", "-l"], ["-s", "-O", "-l"], ["-s"], ["-l"], ["-O"]], ids=lambda f: "".join(f))
+F4_CHUNK = 1 << 25  # -L x5
+F4_FLAGS = [["-O", "-l"], ["-s", "-O", "-l"], ["-s"], ["-l"], ["-O"]]
+
+
+def _f4_file(path):
+    """Three 32 MiB windows and a tail, needles at the window edges and inside the 4 KiB overlaps."""
+    C = F4_CHUNK
+    size = 3 * C + 12345
+    return _big_file(path, size, [1000, C - 4096 + 100, C - 3, 2 * (C - 4096) + 77, size - 6, size - 400])
+
+
+@pytest.mark.parametrize("flags", F4_FLAGS, ids=lambda f: "".join(f))
 def test_host_one_file_over_several_gpus(flags, tmp_path):
     """f4: the windows of ONE file (chunk 32 MiB, 4 KiB overlap) go round 3 'GPUs' as separate batches; stdout is the
     reference's, including the Q3 duplicate in the overlap and -s stopping the FILE after the first printing window
     (grab.cc:232-233) even though later windows were scanned by other lanes."""
-    C = 1 << 25
-    size = 3 * C + 12345
-    needles = [1000, C - 4096 + 100, C - 3, 2 * (C - 4096) + 77, size - 6, size - 400]
+    C = F4_CHUNK
     fn = str(tmp_path / "big.bin")
-    img = _big_file(fn, size, needles)
+    img = _f4_file(fn)
     L5 = ["-L"] * 5
     env = dict(GRAB_B200_NDEV="3", GRAB_B200_BATCH_BYTES="1", GSCAN_DOUBLE_JITTER="1")
     rc, so, se = run(L5 + flags + ["NEEDLE", fn], env=env)
@@ -162,9 +184,7 @@ def test_host_one_file_over_several_gpus(flags, tmp_path):
     want = O.Regex("NEEDLE").grab(img.tobytes(), offsets="-O" in flags, line="-l" not in flags, single="-s" in flags,
                                   chunk_size=C)
     assert so == want
-    if os.path.exists(REF):
-        rcr, ref, _ = run(L5 + flags + ["NEEDLE", fn], binary=REF)
-        assert rcr == 0 and so == ref
+    assert so == base64.b64decode(host_ref()["f4"][" ".join(flags)])
     rc, one, se = run(L5 + flags + ["NEEDLE", fn])
     assert rc == 0 and one == so
 
@@ -235,9 +255,8 @@ def test_host_good_path_then_missing_path(tmp_path):
     assert rc == 255
     assert so == b"a:Match at offset 3\na:Match at offset 13\n"
     assert b"FileGrep::find::stat" in se
-    if os.path.exists(REF):
-        rcr, ref_out, ref_err = run(["-O", "-l", "foo", "a", "nope"], cwd=str(tmp_path), binary=REF)
-        assert (rcr, ref_out) == (rc, so) and ref_err == se
+    ref = host_ref()["good_then_missing"]
+    assert (ref["rc"], base64.b64decode(ref["stdout"])) == (rc, so) and base64.b64decode(ref["stderr"]) == se
 
 
 @pytest.mark.parametrize("flags", [["-r", "-O", "-l"], ["-r", "-l"], ["-r", "-s", "-O", "-l"]], ids=lambda f: "".join(f))

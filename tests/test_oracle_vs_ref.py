@@ -1,6 +1,13 @@
-"""Pins the oracle port to the UNMODIFIED reference binary (oracle/_ref/grab_ref: grab master built against the PCRE2
-shim) on seeded random patterns x random inputs, and to GNU grep -P (same libpcre2) as an independent second opinion.
-CPU only; skipped where the reference binary is not built (it needs /root/reference at build time)."""
+"""Pins the oracle port to the UNMODIFIED reference binary (grab master built against the PCRE2 shim) on seeded random
+patterns x random inputs, and to GNU grep -P (same libpcre2) as an independent second opinion.  CPU only.
+
+The reference's stdout for every (pattern, flags, input) compared here is recorded in tests/golden/ref_stdout.json.gz
+(sha-256 digests, written by tests/golden/make_golden.py from a run of the reference), so the comparison needs neither
+the reference's sources nor its binary."""
+import functools
+import gzip
+import hashlib
+import json
 import os
 import random
 import shutil
@@ -12,15 +19,33 @@ import oracle_py as O
 from test_gpu_random_patterns import gen_pattern
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.path.join(os.path.dirname(HERE), "oracle", "_ref", "grab_ref")
+GOLDEN = os.path.join(HERE, "golden", "ref_stdout.json.gz")
+REF_TIMEOUT_S = 20  # a reference run longer than this was recorded as a timeout: the pattern is not compared
 
-needs_ref = pytest.mark.skipif(not os.path.exists(REF), reason="oracle/_ref/grab_ref not built")
+
+def digest(stdout):
+    return hashlib.sha256(stdout).hexdigest()[:32]
 
 
-def ref_offsets(pattern, path, flags=("-O", "-l")):
-    p = subprocess.run([REF] + list(flags) + [pattern, path], stdout=subprocess.PIPE, stderr=subprocess.PIPE, timeout=20)
-    assert p.returncode == 0, p.stderr
-    return p.stdout
+def input_key(data):
+    return hashlib.sha256(data).hexdigest()[:16]
+
+
+@functools.lru_cache(maxsize=None)
+def recorded():
+    """(pattern, flags, input key) -> digest of the reference's stdout, or None where its run timed out."""
+    with gzip.open(GOLDEN, "rt") as f:
+        return {(pat, tuple(flags), key): d for pat, flags, key, d in json.load(f)}
+
+
+def ref_stdout(pattern, data, flags=("-O", "-l")):
+    """Digest of the reference's stdout for `grab <flags> <pattern> <file holding data>`; raises
+    subprocess.TimeoutExpired where the reference's run timed out when it was recorded."""
+    k = (pattern, tuple(flags), input_key(data))
+    assert k in recorded(), "no recorded reference output for %r: regenerate %s" % (k, GOLDEN)
+    if recorded()[k] is None:
+        raise subprocess.TimeoutExpired(["grab"] + list(flags) + [pattern], REF_TIMEOUT_S)
+    return recorded()[k]
 
 
 def random_inputs(rnd, n):
@@ -32,15 +57,9 @@ def random_inputs(rnd, n):
     return out
 
 
-@needs_ref
-def test_random_patterns_stdout_identical(tmp_path):
+def test_random_patterns_stdout_identical():
     rnd = random.Random(20260924)
     inputs = random_inputs(rnd, 10)
-    paths = []
-    for i, b in enumerate(inputs):
-        p = tmp_path / ("in%d" % i)
-        p.write_bytes(b)
-        paths.append(str(p))
     checked = 0
     for _ in range(150):
         pat = gen_pattern(rnd)
@@ -52,8 +71,8 @@ def test_random_patterns_stdout_identical(tmp_path):
             continue
         try:
             for flags, kw in ((("-O", "-l"), dict(offsets=True, line=False)), ((), dict()), (("-s", "-O"), dict(offsets=True, single=True))):
-                for path, data in zip(paths, inputs):
-                    assert o.grab(data, **kw) == ref_offsets(pat, path, flags), (pat, flags, len(data))
+                for data in inputs:
+                    assert digest(o.grab(data, **kw)) == ref_stdout(pat, data, flags), (pat, flags, len(data))
         except (O.OracleError, subprocess.TimeoutExpired):
             continue  # pathological backtracking: either side hit its match limit / time budget
         checked += 1
@@ -66,8 +85,7 @@ OPTION_PATTERNS = [r"(?U)a+b", r"(?U)a+?b", r"(?U)a{2,}", r"(?U)\w+ ", r"(?U:a+)
                    r"a(?#hello)b", r"(?#c)a|b(?#d)c", r"a(?#x)+b"]
 
 
-@needs_ref
-def test_inline_options_ungreedy_extended_comment(tmp_path):
+def test_inline_options_ungreedy_extended_comment():
     """(?U), (?x) and (?#...) as the reference's PCRE build treats them: identical stdout in all three output modes."""
     rnd = random.Random(5)
     inputs = random_inputs(rnd, 15) + [b"aaab ab\nfoo  bar # x\nabcabc aXb a\nb\n", b"a b c abc a  b\n", b"aab aaab abbc abc\n"]
@@ -76,26 +94,21 @@ def test_inline_options_ungreedy_extended_comment(tmp_path):
         o = O.Regex(pat)
         if o.nullable:
             continue
-        for i, data in enumerate(inputs):
-            path = tmp_path / ("in%d" % i)
-            path.write_bytes(data)
+        for data in inputs:
             for flags, kw in ((("-O", "-l"), dict(offsets=True, line=False)), ((), dict()), (("-s", "-O"), dict(offsets=True, single=True))):
-                assert o.grab(data, **kw) == ref_offsets(pat, str(path), flags), (pat, flags, data)
+                assert digest(o.grab(data, **kw)) == ref_stdout(pat, data, flags), (pat, flags, data)
         checked += 1
     assert checked >= 20
 
 
-@needs_ref
-def test_minlen_quirk_q1_against_reference(tmp_path):
+def test_minlen_quirk_q1_against_reference():
     # the strict '<' of grab.cc:175 for every length around minlen
     for pat, unit in (("abc", b"abc"), ("[ab]{4,}", b"abab"), ("ab|abcd", b"ab")):
         o = O.Regex(pat)
         for reps in range(0, 4):
             for tail in (b"", b"x", b"\n"):
                 data = unit * reps + tail
-                p = tmp_path / "f"
-                p.write_bytes(data)
-                assert o.grab(data, offsets=True, line=False) == ref_offsets(pat, str(p)), (pat, data)
+                assert digest(o.grab(data, offsets=True, line=False)) == ref_stdout(pat, data), (pat, data)
 
 
 @pytest.mark.skipif(shutil.which("grep") is None, reason="no grep")
@@ -123,8 +136,7 @@ def test_second_opinion_gnu_grep_P(tmp_path):
             assert got == want, (pat, data)
 
 
-@needs_ref
-def test_long_lines_line_mode_against_reference(tmp_path):
+def test_long_lines_line_mode_against_reference():
     """Line output on lines longer than the 511 bytes the reference prints behind a match (grab.cc:194-196): the next search
     resumes in the middle of the line -- for class runs possibly in the middle of a run, where PCRE then reports a match at
     the resume point itself.  The resolve pass's chain path for class runs (k_chain_next / k_chain_entry) is built on
@@ -143,9 +155,7 @@ def test_long_lines_line_mode_against_reference(tmp_path):
     for pat in pats:
         o = O.Regex(pat)
         for i, data in enumerate(inputs):
-            path = tmp_path / ("long%d" % i)
-            path.write_bytes(data)
             for flags, kw in (((), dict()), (("-O",), dict(offsets=True)), (("-O", "-l"), dict(offsets=True, line=False))):
-                assert o.grab(data, **kw) == ref_offsets(pat, str(path), flags), (pat, flags, i, len(data))
+                assert digest(o.grab(data, **kw)) == ref_stdout(pat, data, flags), (pat, flags, i, len(data))
                 checked += 1
     assert checked == len(pats) * len(inputs) * 3
