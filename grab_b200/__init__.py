@@ -39,7 +39,7 @@ UNIT_DTYPE = np.dtype([("ptr", "<u8"), ("len", "<u8"), ("base_off", "<u8"), ("fi
 
 class PatternInfo(ctypes.Structure):
     _fields_ = [(n, ctypes.c_int32) for n in ("minlen", "maxlen", "captures", "engine", "n_sequences",
-                                              "n_filter_tests", "filter_anchor", "filter_delta", "scan_kernel", "reserved")]
+                                              "n_filter_tests", "filter_anchor", "filter_delta", "scan_kernel", "scan_variant")]
 
 
 class Stats(ctypes.Structure):

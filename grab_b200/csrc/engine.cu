@@ -344,12 +344,25 @@ extern "C" int gscan_pattern_get_info(const gscan_pattern *p, gscan_pattern_info
 	o->n_filter_tests = p->prog.use_hash ? -(int32_t)p->prog.hash_slots : (int32_t)p->prog.tests.size();
 	o->filter_anchor = p->prog.anchor;
 	o->filter_delta = p->prog.delta;
-	o->reserved = 0;
+	o->scan_variant = 0;
 	if (p->prog.kind == ENGINE_NONE || (p->prog.use_vm && p->prog.vm_dense)) o->scan_kernel = GSCAN_KERNEL_NONE;
 	else if (p->prog.kind == ENGINE_RUN) o->scan_kernel = GSCAN_KERNEL_RUN;
 	else if (p->prog.use_hash) o->scan_kernel = GSCAN_KERNEL_HASH;
 	else if (p->fixed.b_engine) o->scan_kernel = GSCAN_KERNEL_BALANCED;
 	else o->scan_kernel = p->fixed.stage1_triples ? GSCAN_KERNEL_TRIPLE : GSCAN_KERNEL_PAIR;
+	// what launch_scan_fixed / launch_scan_hash / launch_scan_run dispatch on (layout: include/gscan.h)
+	if (o->scan_kernel == GSCAN_KERNEL_RUN) {
+		const RunParams &R = p->run;
+		o->scan_variant = (int32_t)(R.nlo | R.nhi << 4 | R.nfold << 6 | (R.run_min > 17u ? GSCAN_SV_RUN_LONG : 0u));
+	} else if (o->scan_kernel == GSCAN_KERNEL_HASH) {
+		const HashParams &H = p->hash;
+		o->scan_variant = (int32_t)(H.hash_len | (H.pre_enable ? GSCAN_SV_HASH_SPARSE : 0u) | (H.stride / 4u) << 3);
+	} else if (o->scan_kernel != GSCAN_KERNEL_NONE) {
+		const FixedParams &F = p->fixed;
+		o->scan_variant = (int32_t)(F.ntests | (uint32_t)p->prog.delta << 4 | (F.exact ? GSCAN_SV_EXACT : 0u) |
+		                            (F.b_engine ? GSCAN_SV_BALANCED : 0u) | (F.b_aligned ? GSCAN_SV_ALIGNED : 0u) |
+		                            (F.stage1_triples ? GSCAN_SV_STAGE1_TRIPLES : 0u) | F.n2 << 11 | (F.exact3 ? GSCAN_SV_EXACT3 : 0u));
+	}
 	return 0;
 }
 

@@ -76,8 +76,35 @@ typedef struct gscan_pattern_info {
 	int32_t filter_anchor; /* byte of the pattern the SWAR filter is anchored on */
 	int32_t filter_delta;  /* distance to the second filter byte (0: single-byte filter) */
 	int32_t scan_kernel;   /* GSCAN_KERNEL_* below: which scan-kernel family serves the pattern */
-	int32_t reserved;
+	int32_t scan_variant;  /* the values the scan-kernel launch dispatches on (bit layout below), 0 for GSCAN_KERNEL_NONE */
 } gscan_pattern_info;
+
+/* scan_variant: raw values, not template arguments (the launcher maps e.g. 5 tests to the 6-test instantiation).
+ *   PAIR / TRIPLE / BALANCED  bits 0-3  n_filter_tests (0..8)      bits 4-6  filter_delta (0..4)
+ *                             bit  7    every pair test exact      bit  8    balanced pair filter
+ *                             bit  9    balanced: one third-byte test per pair test (aligned stage 2)
+ *                             bit 10    byte-triple stage-1 filter bits 11-15 third-byte tests (0..16)
+ *                             bit 16    every triple test exact
+ *   RUN                       bits 0-3  byte ranges below 0x80     bits 4-5  ranges in 0x80-0xff (0..2)
+ *                             bit  6    one [A-Z]/[a-z]-style range pair folded into one test
+ *                             bit  7    run minimum above 17 (bytes 17.. confirmed from global memory)
+ *   HASH                      bits 0-1  key bytes (2 or 3)         bit  2    sparse path possible (class prefilter)
+ *                             bits 3-8  table copies in shared memory (32, 16 or 1) */
+#define GSCAN_SV_TESTS(v) ((v) & 15)
+#define GSCAN_SV_DELTA(v) (((v) >> 4) & 7)
+#define GSCAN_SV_EXACT 0x80
+#define GSCAN_SV_BALANCED 0x100
+#define GSCAN_SV_ALIGNED 0x200
+#define GSCAN_SV_STAGE1_TRIPLES 0x400
+#define GSCAN_SV_TRIPLES(v) (((v) >> 11) & 31)
+#define GSCAN_SV_EXACT3 0x10000
+#define GSCAN_SV_RUN_NLO(v) ((v) & 15)
+#define GSCAN_SV_RUN_NHI(v) (((v) >> 4) & 3)
+#define GSCAN_SV_RUN_FOLD 0x40
+#define GSCAN_SV_RUN_LONG 0x80
+#define GSCAN_SV_HASH_LEN(v) ((v) & 3)
+#define GSCAN_SV_HASH_SPARSE 0x4
+#define GSCAN_SV_HASH_COPIES(v) (((v) >> 3) & 63)
 
 #define GSCAN_KERNEL_NONE 0
 #define GSCAN_KERNEL_PAIR 1     /* byte-pair SWAR filter (single literals: the HBM-bound kernel) */

@@ -350,7 +350,8 @@ def gen_ref_stdout():
 
     T.ref_stdout = run
     for name in ("test_random_patterns_stdout_identical", "test_inline_options_ungreedy_extended_comment",
-                 "test_minlen_quirk_q1_against_reference", "test_long_lines_line_mode_against_reference"):
+                 "test_minlen_quirk_q1_against_reference", "test_long_lines_line_mode_against_reference",
+                 "test_binary_inputs_stdout_identical"):
         getattr(T, name)()
     return [[pat, list(flags), key, d] for (pat, flags, key), d in sorted(rows.items(), key=lambda kv: json.dumps(kv[0]))]
 

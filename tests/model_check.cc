@@ -474,6 +474,24 @@ int main(int argc, char **argv)
 		if (k >= 3) b[ln / 2] = '\n';
 		subjects.push_back(b);
 	}
+	// binary subjects: uniform bytes, the ASCII alphabets with bit 7 or bit 5 flipped (what SWAR filters that ignore a bit
+	// let through), and text with NUL bytes and a run of NULs
+	for (int k = 0; k < 40; k++) {
+		const char *al = alphas[k % 6];
+		const size_t na = strlen(al), ln = (size_t)lens[(k * 7) % 13] + (k & 1) * 200;
+		std::vector<uint8_t> b(ln);
+		for (auto &c : b) {
+			const uint8_t a = (uint8_t)al[rnd() % na];
+			switch (k / 10) {
+			case 0: c = (uint8_t)rnd(); break;
+			case 1: c = rnd() % 3 ? a : (uint8_t)(a ^ 0x80); break;
+			case 2: c = rnd() % 3 ? a : (uint8_t)(a ^ 0x20); break;
+			default: c = rnd() % 4 ? a : 0; break;
+			}
+		}
+		if (k / 10 == 3) for (size_t i = ln / 3; i < ln / 3 + ln / 4; i++) b[i] = 0;
+		subjects.push_back(b);
+	}
 	int n_dense = 0, n_pat = 0, n_served = 0, n_vm = 0, n_cmp = 0, n_walk = 0, n_limit = 0, bad = 0, n_strict = 0;
 	while (std::getline(f, pat)) {
 		if (pat.empty()) continue;

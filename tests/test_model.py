@@ -6,6 +6,7 @@ import subprocess
 
 import test_gpu_random_patterns as R
 import test_gpu_parity as P
+from test_scan_variants import VARIANTS
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
@@ -31,6 +32,7 @@ def test_compiled_programs_match_the_oracle(tmp_path):
     import json
     kat = json.load(open(os.path.join(HERE, "golden", "kat.json")))
     pats += sorted({c["pattern"] for c in kat["cases"]})  # the reference's recorded cases
+    pats += [p for key in sorted(VARIANTS, key=str) for p in VARIANTS[key]]  # every scan-kernel instantiation, high bytes and NUL
     (tmp_path / "patterns.txt").write_text("\n".join(p for p in pats if "\n" not in p) + "\n")
     exe = str(tmp_path / "model_check")
     subprocess.run(["gcc", "-O2", "-c", os.path.join(ROOT, "oracle", "grab_oracle.c"), "-o", str(tmp_path / "oracle.o")], check=True)

@@ -136,6 +136,25 @@ def test_second_opinion_gnu_grep_P(tmp_path):
             assert got == want, (pat, data)
 
 
+def test_binary_inputs_stdout_identical():
+    """Every pattern of test_scan_variants.VARIANTS (high bytes, NUL, (?i) next to bytes >= 0x80 -- which PCRE's C locale does
+    not fold) on seeded binary inputs of test_gpu_binary's generators: the oracle the GPU tests trust holds on binary input."""
+    import numpy as np
+    from test_gpu_binary import small_units
+    from test_scan_variants import VARIANTS
+    checked = 0
+    for key in sorted(VARIANTS, key=str):
+        for pat in VARIANTS[key]:
+            o = O.Regex(pat)
+            units = small_units(pat, random.Random("ref|" + pat))
+            for u in (units[62], units[-1]):  # 63 bytes of text salted with high bytes, 4096 uniform bytes
+                data = np.asarray(u, dtype=np.uint8).tobytes()
+                for flags, kw in ((("-O", "-l"), dict(offsets=True, line=False)), ((), dict()), (("-s", "-O"), dict(offsets=True, single=True))):
+                    assert digest(o.grab(data, **kw)) == ref_stdout(pat, data, flags), (pat, flags, len(data))
+                    checked += 1
+    assert checked >= 300
+
+
 def test_long_lines_line_mode_against_reference():
     """Line output on lines longer than the 511 bytes the reference prints behind a match (grab.cc:194-196): the next search
     resumes in the middle of the line -- for class runs possibly in the middle of a run, where PCRE then reports a match at
